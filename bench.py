@@ -3,7 +3,8 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4] [--regime peaky|diffuse]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...        # CPU arm: the unmodified Python reference over a fork pool
-                                                # (baseline/_ref; LM workloads: the oracle C++ port)
+                                                # (oracle/_ref; LM workloads: the oracle C++ port)
+    python bench.py --dump-outputs DIR ...      # also write the last timed step's results to DIR/*.npy
 
 A "step" is one decode_batch() pass over one batch of synthetic logits.  `value` is frames/s
 with the batch already resident in HBM (device pointers handed to the C ABI); `e2e` is the same
@@ -19,6 +20,7 @@ Prints ONE JSON line on rank 0.  Besides the headline (C2) the line carries
                    broadcast of the LM blob, checked against rank 0's single-GPU decode of the same list.
 """
 import argparse
+import io
 import json
 import os
 import statistics
@@ -221,11 +223,11 @@ def port_arm(wl, spec, kw, xs, beam, hot, target_cpu_seconds=20.0, min_utts=0, w
                       "%d threads, %.1f s" % (n, spec["T"], cores, dt)}, texts, n
 
 
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 
 
 def pyref_available(spec):
-    """The unmodified reference (pip-installed from /root/reference into baseline/_ref, which travels to the GPU box)
+    """The unmodified reference (pip-installed into oracle/_ref by build(), see oracle.install_reference)
     can be timed for workloads without a language model: its only missing hard dependency is then pygtrie's import,
     served by the stand-in under oracle/refshim.  LM workloads would run on the pure-Python kenlm stand-in, which
     would handicap the reference -- they are timed on the C++ port instead."""
@@ -288,7 +290,7 @@ def reference_main(args, spec, B, beam):
                 vals.append(n * T / dt)
         ref.close()
         kind = "reference"
-        what = ("%d utterances x T=%d of the same workload, the UNMODIFIED Python reference (baseline/_ref, pyctcdecode 0.6.0) "
+        what = ("%d utterances x T=%d of the same workload, the UNMODIFIED Python reference (oracle/_ref, pyctcdecode 0.6.0) "
                 "through decode_batch over a fork Pool(%d), %.1f s per step" % (n, T, cores, n * T / vals[-1]))
     else:
         vals, info = [], None
@@ -378,6 +380,58 @@ class Stepper:
         return total, tms, out
 
 
+DUMP_LIMIT = 64_000_000      # bytes of .npy files (64 MB)
+
+
+def _codepoints(texts):
+    """strings -> [N, longest] float32 Unicode code points (exact: every code point is below 2^24), padded with -1"""
+    arr = np.full((len(texts), max([len(t) for t in texts], default=0)), -1.0, np.float32)
+    for i, t in enumerate(texts):
+        arr[i, :len(t)] = [ord(c) for c in t]
+    return arr
+
+
+def output_arrays(call, out, keep):
+    """What `call` returned for the utterances `keep`, one row per transcript: decode_batch -> `text`;
+    decode_beams_batch -> every beam's `text`, `logit_score`, `lm_score` and `word_frames` (start and end frame of each
+    word, padded with -1).  `utterance` is the batch index of each row."""
+    if call == "decode_batch":
+        return {"utterance": keep.astype(np.float64), "text": _codepoints([out[i] for i in keep])}
+    beams = [(i, b) for i in keep for b in out[i]]
+    frames = np.full((len(beams), max([len(b.text_frames) for _, b in beams], default=0), 2), -1.0, np.float32)
+    for r, (_, b) in enumerate(beams):
+        for w, (_, span) in enumerate(b.text_frames):
+            frames[r, w] = span
+    return {"utterance": np.array([i for i, _ in beams], np.float64), "text": _codepoints([b.text for _, b in beams]),
+            "logit_score": np.array([b.logit_score for _, b in beams], np.float64),
+            "lm_score": np.array([b.lm_score for _, b in beams], np.float64), "word_frames": frames}
+
+
+def _npy_files(arrays):
+    """{name: the bytes of name.npy, header included}"""
+    files = {}
+    for name, arr in arrays.items():
+        buf = io.BytesIO()
+        np.save(buf, arr)
+        files[name] = buf.getvalue()
+    return files
+
+
+def dump_outputs(path, call, out):
+    """DIR/<name>.npy of output_arrays() for the whole batch or, above DUMP_LIMIT bytes of files, for a fixed sample
+    of it: a prefix of a seeded permutation, halved until the files fit"""
+    keep = np.arange(len(out))
+    perm = np.random.default_rng(0).permutation(len(out))
+    files = _npy_files(output_arrays(call, out, keep))
+    while sum(len(b) for b in files.values()) > DUMP_LIMIT and len(keep) > 1:
+        keep = np.sort(perm[:len(keep) // 2])
+        files = _npy_files(output_arrays(call, out, keep))
+    os.makedirs(path, exist_ok=True)
+    for name, data in files.items():
+        with open(os.path.join(path, name + ".npy"), "wb") as fh:
+            fh.write(data)
+
+
 def load_peaks():
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as fh:
@@ -461,7 +515,7 @@ def streaming_entry(torch, pkg, name, spec, n_streams, chunk=50, beam=100):
     informational: every chunk ends with _finalize_beams (sort, trim, prune), so the reference's own streaming result
     differs from its one-shot decode on a few percent of the utterances too; parity of the streaming path is what the
     22 reference-generated streaming goldens and `cpu_baseline.final_text_equals_b200` check.  CPU figure: the unmodified Python reference's own partial_decode_beams on
-    one stream (workloads without a language model, when baseline/_ref is present)."""
+    one stream (workloads without a language model, when oracle/_ref is present)."""
     t_start = time.perf_counter()
     wl, kw, _ = workload_objects(spec)
     T = spec["T"]
@@ -601,7 +655,13 @@ def main():
     ap.add_argument("--ref-port", action="store_true", help="reference arm: time the oracle C++ port even where the Python reference can run")
     ap.add_argument("--ref-seconds", type=float, default=0.0, help="reference arm: target seconds of one step (default: sized from --steps)")
     ap.add_argument("--emit-texts", action="store_true", help="reference arm: add the transcripts of the last step to the JSON line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step of the headline call returned (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -665,6 +725,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     e2e_total, e2e_tms, texts_e2e = st.timed(st.step_host, args.steps, args.warmup, flush)   # the same W warm-up steps as the device-resident arm
     assert texts == texts_e2e
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, args.call, texts)
     if args.call != "decode_batch":
         texts = [beams[0].text if beams else "" for beams in texts]
 

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY (build container only: needs /root/reference).
 
-Generates tests/golden/{cases.json,arrays.npz} by running the UNMODIFIED reference
+Generates tests/golden/{cases.json,arrays.npz,arrays_large.npz} by running the UNMODIFIED reference
 (/root/reference/pyctcdecode, imported with the kenlm / pygtrie stand-ins of oracle/refshim)
 on (a) the reference's own test fixtures (tests/test_decoder.py:186-223, sample_data/) and
 (b) small seeded synthetic utterances (tests/synth.py).  The GPU box has no /root/reference,
@@ -27,7 +27,7 @@ logging.disable(logging.CRITICAL)
 from pyctcdecode import build_ctcdecoder  # noqa: E402  (the reference)
 from pyctcdecode.alphabet import Alphabet  # noqa: E402
 
-from tests import synth  # noqa: E402
+from tests import goldens, synth  # noqa: E402
 
 REF_TESTS = "/root/reference/pyctcdecode/tests"
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -171,7 +171,7 @@ def main():
         al = Alphabet.build_alphabet(labels)
         alpha_cases.append({"labels": labels, "normalized": al.labels, "is_bpe": al.is_bpe})
 
-    np.savez_compressed(os.path.join(OUT, "arrays.npz"), **arrays)
+    goldens.save_arrays(OUT, arrays)
     with open(os.path.join(OUT, "cases.json"), "w", encoding="utf-8") as fh:
         json.dump({"toy_arpa": toy_arpa, "cases": cases, "alphabet": alpha_cases,
                    "generator": "oracle/gen_golden.py", "reference": "pyctcdecode 0.6.0 @ afecb676, numpy %s" % np.__version__},

@@ -27,7 +27,7 @@ from pyctcdecode import BeamSearchDecoderCTC, LanguageModel  # noqa: E402  (the 
 from pyctcdecode.language_model import MultiLanguageModel  # noqa: E402
 from pyctcdecode.alphabet import Alphabet  # noqa: E402
 
-from tests import synth  # noqa: E402
+from tests import goldens, synth  # noqa: E402
 
 REF_TESTS = "/root/reference/pyctcdecode/tests"
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -57,7 +57,7 @@ def build_models(specs, toy):
 
 
 def main():
-    base = dict(np.load(os.path.join(OUT, "arrays.npz")))
+    base = goldens.load_arrays(OUT)
     toy = os.path.join(REF_TESTS, "sample_data", "bugs_bunny_kenlm.arpa")
     SAMPLE_LABELS = [" ", "b", "g", "n", "s", "u", "y", ""]
     arrays, cases = {}, []

@@ -27,7 +27,7 @@ logging.disable(logging.CRITICAL)
 from pyctcdecode import build_ctcdecoder  # noqa: E402  (the reference)
 from pyctcdecode.language_model import HotwordScorer  # noqa: E402
 
-from tests import synth  # noqa: E402
+from tests import goldens, synth  # noqa: E402
 
 REF_TESTS = "/root/reference/pyctcdecode/tests"
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -41,7 +41,7 @@ def beams_json(beams):
 
 
 def main():
-    base = dict(np.load(os.path.join(OUT, "arrays.npz")))
+    base = goldens.load_arrays(OUT)
     extra, cases = {}, []
     toy = os.path.join(REF_TESTS, "sample_data", "bugs_bunny_kenlm.arpa")
     SAMPLE_LABELS = [" ", "b", "g", "n", "s", "u", "y", ""]

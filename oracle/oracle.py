@@ -17,6 +17,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_PATH = os.path.join(_HERE, "liboracle.so")
+REF_DIR = os.path.join(_HERE, "_ref")
 _lib = None
 
 
@@ -26,6 +27,33 @@ def build(force=False):
     if force or not os.path.exists(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < os.path.getmtime(src):
         subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "liboracle.so"])
     return _LIB_PATH
+
+
+def install_reference():
+    """pip-install the UNMODIFIED reference package into oracle/_ref (git-ignored) for bench.py's reference arm.
+    The checkout of kensho-technologies/pyctcdecode 0.6.0 is named by $PYCTCDECODE_REFERENCE; without it nothing is
+    installed and bench.py times the C++ port instead.  Installed from a copy: pip builds in the source tree.
+    Best effort: when the install cannot run (no pip, no setuptools, not a checkout) it warns and installs nothing,
+    since the product and its tests do not need it."""
+    import shutil
+    import sys
+    import tempfile
+    src = os.environ.get("PYCTCDECODE_REFERENCE")
+    if not src or os.path.isdir(os.path.join(REF_DIR, "pyctcdecode")):
+        return
+    if not os.path.isdir(os.path.join(src, "pyctcdecode")):
+        print("oracle/_ref: PYCTCDECODE_REFERENCE=%s is not a pyctcdecode checkout; not installed" % src, file=sys.stderr)
+        return
+    with tempfile.TemporaryDirectory() as tmp:
+        copy = os.path.join(tmp, "reference")
+        shutil.copytree(src, copy, ignore=shutil.ignore_patterns(".git"))
+        cmd = [sys.executable, "-m", "pip", "install", "--no-index", "--no-build-isolation", "--no-deps", "--no-cache-dir",
+               "--quiet", "--target", REF_DIR, copy]
+        log = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
+    if log.returncode != 0:
+        shutil.rmtree(REF_DIR, ignore_errors=True)       # no partial install for bench.py to find
+        print("oracle/_ref: installing the reference failed, bench.py times the C++ port:\n" + log.stdout[-2000:],
+              file=sys.stderr)
 
 
 def lib():

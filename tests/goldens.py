@@ -1,7 +1,6 @@
 """Loader for tests/golden (vectors produced by oracle/gen_golden.py from the unmodified reference)."""
 import json
 import os
-import tempfile
 
 import numpy as np
 
@@ -10,15 +9,30 @@ from tests import synth
 HERE = os.path.dirname(os.path.abspath(__file__))
 _cache = {}
 
+# The arrays of cases.json are stored in two files, so that neither is above 1 MB: the largest logits in the second.
+ARRAY_FILES = ("arrays.npz", "arrays_large.npz")
+LARGE_ARRAYS = ("syn_C_bpe_0", "syn_C_bpe_4gram_1", "syn_C_bpe_4gram_3")
+
+
+def load_arrays(directory=os.path.join(HERE, "golden")):
+    arrays = {}
+    for name in ARRAY_FILES:
+        arrays.update(np.load(os.path.join(directory, name)))
+    return arrays
+
+
+def save_arrays(directory, arrays):
+    large = {k: v for k, v in arrays.items() if k in LARGE_ARRAYS}
+    np.savez_compressed(os.path.join(directory, ARRAY_FILES[0]), **{k: v for k, v in arrays.items() if k not in large})
+    np.savez_compressed(os.path.join(directory, ARRAY_FILES[1]), **large)
+
 
 def load():
     if "g" not in _cache:
         with open(os.path.join(HERE, "golden", "cases.json"), encoding="utf-8") as fh:
             meta = json.load(fh)
-        arrays = dict(np.load(os.path.join(HERE, "golden", "arrays.npz")))
-        d = os.path.join(tempfile.gettempdir(), "b200ctc_synth")
-        os.makedirs(d, exist_ok=True)
-        toy = os.path.join(d, "bugs_bunny_kenlm.arpa")
+        arrays = load_arrays()
+        toy = os.path.join(synth.cache_dir(), "bugs_bunny_kenlm.arpa")
         with open(toy, "w", encoding="utf-8") as fh:
             fh.write(meta["toy_arpa"])
         _cache["g"] = {"meta": meta, "arrays": arrays, "toy_arpa": toy, "workloads": {}}

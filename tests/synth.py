@@ -138,11 +138,17 @@ def write_synthetic_arpa(path, words, probs, order=3, seed=2, succ_lo=4, succ_hi
     return {"vocab": vocab, "levels": levels, "widx": widx}
 
 
-def cached_arpa(n_words, letters, order, seed=1, tag=""):
-    """Create (or reuse) a synthetic ARPA under the system temp dir. Returns (path, words, probs, tables)."""
-    key = hashlib.sha1(("%d|%s|%d|%d|%s|v3" % (n_words, "".join(letters), order, seed, tag)).encode()).hexdigest()[:12]
-    d = os.path.join(tempfile.gettempdir(), "b200ctc_synth")
+def cache_dir():
+    """Per-user directory under the system temp dir: on a shared machine another user's directory is not writable."""
+    d = os.path.join(tempfile.gettempdir(), "b200ctc_synth-%d" % os.getuid())
     os.makedirs(d, exist_ok=True)
+    return d
+
+
+def cached_arpa(n_words, letters, order, seed=1, tag=""):
+    """Create (or reuse) a synthetic ARPA under cache_dir(). Returns (path, words, probs, tables)."""
+    key = hashlib.sha1(("%d|%s|%d|%d|%s|v3" % (n_words, "".join(letters), order, seed, tag)).encode()).hexdigest()[:12]
+    d = cache_dir()
     path = os.path.join(d, "lm_%s.arpa" % key)
     words, probs = make_word_list(n_words, letters, seed=seed)
     tmp = path + ".tmp%d" % os.getpid()
