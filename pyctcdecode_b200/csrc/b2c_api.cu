@@ -290,44 +290,23 @@ B2C_HD void b2c_beam_block(const B2cBeamArgs& A, int slot, u8* smem) {
 // Each variant exists with the label table resident in shared memory (alphabets of up to B2C_FAST_LT labels: runs of
 // in-place frames enabled) and with per-frame label staging (larger alphabets).
 #define B2C_FAST_LT 64
-typedef B2cFastSmem<128, 1024, B2C_FAST_LT> B2cFastSmemA;      // 2 CTAs per SM
-typedef B2cFastSmem<128, 512, B2C_FAST_LT> B2cFastSmemB;       // 3 CTAs per SM
-typedef B2cFastSmem<128, 256, B2C_FAST_LT> B2cFastSmemC;       // 4 CTAs per SM
-// variant 3 is the LEAN one: a one-warp CTA with 32 beam slots and 128 candidates for workloads where few beams stay
-// alive (language model): 8 CTAs per SM; an utterance that needs more is handed back and decoded by a full variant
-typedef B2cFastSmem<32, 128, B2C_FAST_LT> B2cFastSmemL;
-typedef B2cFastSmem<32, 128, 0> B2cFastSmemL0;
-static const u32 kV5Cap[4] = {1024, 512, 256, 128};
-static const int kV5Occ[4] = {2, 3, 4, 8};
-static const int kV5Threads[4] = {128, 128, 128, 32};
+typedef B2cFastSmem<1024, B2C_FAST_LT> B2cFastSmemA;      // 2 CTAs per SM
+typedef B2cFastSmem<512, B2C_FAST_LT> B2cFastSmemB;       // 3 CTAs per SM
+typedef B2cFastSmem<256, B2C_FAST_LT> B2cFastSmemC;       // 4 CTAs per SM
+static const u32 kV5Cap[3] = {1024, 512, 256};
+static const int kV5Occ[3] = {2, 3, 4};
 // [variant][0: staged labels, 1: resident table]
-static const size_t kV5Smem[4][2] = {{sizeof(B2cFastSmem<128, 1024, 0>), sizeof(B2cFastSmemA)},
-                                     {sizeof(B2cFastSmem<128, 512, 0>), sizeof(B2cFastSmemB)},
-                                     {sizeof(B2cFastSmem<128, 256, 0>), sizeof(B2cFastSmemC)},
-                                     {sizeof(B2cFastSmemL0), sizeof(B2cFastSmemL)}};
-static_assert(8 * (sizeof(B2cFastSmemL) + 1024) <= 228 * 1024, "lean variant: 8 CTAs per SM");
+static const size_t kV5Smem[3][2] = {{sizeof(B2cFastSmem<1024, 0>), sizeof(B2cFastSmemA)},
+                                     {sizeof(B2cFastSmem<512, 0>), sizeof(B2cFastSmemB)},
+                                     {sizeof(B2cFastSmem<256, 0>), sizeof(B2cFastSmemC)}};
 // bytes a CTA parks between two chunked launches: everything in front of the per-frame candidate scratch
-typedef B2cFastSmem<128, 1024, 0> B2cFastSmemA0;
-typedef B2cFastSmem<128, 512, 0> B2cFastSmemB0;
-typedef B2cFastSmem<128, 256, 0> B2cFastSmemC0;
-static const size_t kV5Save[4][2] = {{offsetof(B2cFastSmemA0, ckey), offsetof(B2cFastSmemA, ckey)},
+typedef B2cFastSmem<1024, 0> B2cFastSmemA0;
+typedef B2cFastSmem<512, 0> B2cFastSmemB0;
+typedef B2cFastSmem<256, 0> B2cFastSmemC0;
+static const size_t kV5Save[3][2] = {{offsetof(B2cFastSmemA0, ckey), offsetof(B2cFastSmemA, ckey)},
                                      {offsetof(B2cFastSmemB0, ckey), offsetof(B2cFastSmemB, ckey)},
-                                     {offsetof(B2cFastSmemC0, ckey), offsetof(B2cFastSmemC, ckey)},
-                                     {offsetof(B2cFastSmemL0, ckey), offsetof(B2cFastSmemL, ckey)}};
+                                     {offsetof(B2cFastSmemC0, ckey), offsetof(B2cFastSmemC, ckey)}};
 #define B2C_PIPE_CHUNKS 4
-// Features that are ON by default only once a GPU run has validated them (the environment overrides either way:
-// B200CTC_PIPELINE=0/1, B200CTC_LEAN=0/1; read at every call so that tests can switch them).
-#ifndef B2C_DEFAULT_PIPELINE
-#define B2C_DEFAULT_PIPELINE 1
-#endif
-#ifndef B2C_DEFAULT_LEAN
-#define B2C_DEFAULT_LEAN 0
-#endif
-static bool env_switch(const char* name, bool dflt) {
-    const char* e = std::getenv(name);
-    if (!e || !*e) return dflt;
-    return !(e[0] == '0' && e[1] == 0);
-}
 #define B2C_E_RETRY_PLAIN (-1000)     // internal: the pipelined attempt must be redone as a plain call
 static_assert(2 * (sizeof(B2cFastSmemA) + 1024) <= 228 * 1024, "variant A: 2 CTAs per SM");
 static_assert(3 * (sizeof(B2cFastSmemB) + 1024) <= 228 * 1024, "variant B: 3 CTAs per SM");
@@ -368,10 +347,10 @@ B2C_HD void b2c_widen_range(const u16* src, float* dst, u64 begin, u64 end, u64 
 __global__ void __launch_bounds__(256) b2c_widen_kernel(const u16* src, float* dst, u64 n, int bf16) {
     b2c_widen_range(src, dst, static_cast<u64>(blockIdx.x) * blockDim.x + threadIdx.x, n, static_cast<u64>(gridDim.x) * blockDim.x, bf16);
 }
-template <int WC, int CAP, int OCC, int LT>
-__global__ void __launch_bounds__(WC, OCC) b2c_beam_fast_kernel(const B2cBeamArgs A) {
+template <int CAP, int OCC, int LT>
+__global__ void __launch_bounds__(B2C_FAST_W, OCC) b2c_beam_fast_kernel(const B2cBeamArgs A) {
     extern __shared__ __align__(16) u8 b2c_smem[];
-    b2c_beam_block_fast<WC, CAP, LT>(A, static_cast<int>(blockIdx.x), b2c_smem);
+    b2c_beam_block_fast<CAP, LT>(A, static_cast<int>(blockIdx.x), b2c_smem);
 }
 // device-resident utterances that are not adjacent in memory (a padded [B, T, V] batch with lengths, a list
 // of separate tensors): ONE launch packs their valid rows, instead of one cudaMemcpyAsync per utterance
@@ -575,8 +554,6 @@ struct b2c_decoder {
     int hint_beam = 0, hint_lm = 0, hint_hot = 0, hint_prune = 0;
     u32 hint_over[6] = {0, 0, 0, 0, 0, 0};
     u32 hint_frames = 0;
-    u32 hint_wide_utts = 0, hint_utts = 0;   // utterances of the previous call a one-warp CTA could not have held / all
-    bool lean_bad = false;                   // the lean variant handed back too many utterances for this configuration
 };
 
 struct BeamRes {
@@ -746,34 +723,30 @@ static int launch_beam(b2c_decoder* d, const B2cBeamArgs& A, int slots, bool fas
     std::vector<u8> smem(A.L.smem_bytes + 64);
     const bool table = A.P.V <= B2C_FAST_LT;
     for (int s = 0; s < slots; ++s) {
-        if (v5 == 0 && table) b2c_beam_block_fast<128, 1024, B2C_FAST_LT>(A, s, smem.data());
-        else if (v5 == 0) b2c_beam_block_fast<128, 1024, 0>(A, s, smem.data());
-        else if (v5 == 1 && table) b2c_beam_block_fast<128, 512, B2C_FAST_LT>(A, s, smem.data());
-        else if (v5 == 1) b2c_beam_block_fast<128, 512, 0>(A, s, smem.data());
-        else if (v5 == 2 && table) b2c_beam_block_fast<128, 256, B2C_FAST_LT>(A, s, smem.data());
-        else if (v5 == 2) b2c_beam_block_fast<128, 256, 0>(A, s, smem.data());
-        else if (v5 == 3 && table) b2c_beam_block_fast<32, 128, B2C_FAST_LT>(A, s, smem.data());
-        else if (v5 == 3) b2c_beam_block_fast<32, 128, 0>(A, s, smem.data());
+        if (v5 == 0 && table) b2c_beam_block_fast<1024, B2C_FAST_LT>(A, s, smem.data());
+        else if (v5 == 0) b2c_beam_block_fast<1024, 0>(A, s, smem.data());
+        else if (v5 == 1 && table) b2c_beam_block_fast<512, B2C_FAST_LT>(A, s, smem.data());
+        else if (v5 == 1) b2c_beam_block_fast<512, 0>(A, s, smem.data());
+        else if (v5 == 2 && table) b2c_beam_block_fast<256, B2C_FAST_LT>(A, s, smem.data());
+        else if (v5 == 2) b2c_beam_block_fast<256, 0>(A, s, smem.data());
         else if (fast) b2c_beam_block<true>(A, s, smem.data());
         else b2c_beam_block<false>(A, s, smem.data());
     }
 #else
     const int smem = static_cast<int>(A.L.smem_bytes);
-#define B2C_LAUNCH_V5(WC, CAP, OCC, LT)                                                                                 \
+#define B2C_LAUNCH_V5(CAP, OCC, LT)                                                                                     \
     do {                                                                                                               \
-        CUDA_OK(cudaFuncSetAttribute(b2c_beam_fast_kernel<WC, CAP, OCC, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-        b2c_beam_fast_kernel<WC, CAP, OCC, LT><<<slots, WC, A.L.smem_bytes, stream>>>(A);                             \
+        CUDA_OK(cudaFuncSetAttribute(b2c_beam_fast_kernel<CAP, OCC, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+        b2c_beam_fast_kernel<CAP, OCC, LT><<<slots, B2C_FAST_W, A.L.smem_bytes, stream>>>(A);                         \
     } while (0)
     if (v5 >= 0) {
         const bool table = A.P.V <= B2C_FAST_LT;
-        if (v5 == 0 && table) B2C_LAUNCH_V5(128, 1024, 2, B2C_FAST_LT);
-        else if (v5 == 0) B2C_LAUNCH_V5(128, 1024, 2, 0);
-        else if (v5 == 1 && table) B2C_LAUNCH_V5(128, 512, 3, B2C_FAST_LT);
-        else if (v5 == 1) B2C_LAUNCH_V5(128, 512, 3, 0);
-        else if (v5 == 2 && table) B2C_LAUNCH_V5(128, 256, 4, B2C_FAST_LT);
-        else if (v5 == 2) B2C_LAUNCH_V5(128, 256, 4, 0);
-        else if (table) B2C_LAUNCH_V5(32, 128, 8, B2C_FAST_LT);
-        else B2C_LAUNCH_V5(32, 128, 8, 0);
+        if (v5 == 0 && table) B2C_LAUNCH_V5(1024, 2, B2C_FAST_LT);
+        else if (v5 == 0) B2C_LAUNCH_V5(1024, 2, 0);
+        else if (v5 == 1 && table) B2C_LAUNCH_V5(512, 3, B2C_FAST_LT);
+        else if (v5 == 1) B2C_LAUNCH_V5(512, 3, 0);
+        else if (table) B2C_LAUNCH_V5(256, 4, B2C_FAST_LT);
+        else B2C_LAUNCH_V5(256, 4, 0);
         CUDA_OK(cudaGetLastError());
         return 0;
     }
@@ -1329,7 +1302,7 @@ static int decode_batch_locked(b2c_decoder_t* d, const void* const* logits, cons
     // call that turns out to hold probabilities is redone as a plain call (B2C_E_RETRY_PLAIN).
     const bool hint_ok = d->hint_valid && d->hint_beam == opts->beam_width && d->hint_lm == (P.lm.order > 0 ? 1 : 0) &&
                          d->hint_hot == (P.n_hot > 0 ? 1 : 0) && d->hint_prune == P.prune_history && d->hint_frames > 0;
-    const bool no_pipe = std::getenv("B200CTC_NO_PIPELINE") != nullptr || !env_switch("B200CTC_PIPELINE", B2C_DEFAULT_PIPELINE != 0);
+    const bool no_pipe = std::getenv("B200CTC_NO_PIPELINE") != nullptr;
     bool pipe_candidate = allow_pipe && !no_pipe && !is_device && !half_in && T_max >= 8 * B2C_TILE_ROWS &&
                           !streaming && n_lm == 1 && opts->beam_width <= 128 && hint_ok && !d->pipe_refused;
     for (int i = 0; i < n_utts && pipe_candidate; ++i)
@@ -1531,11 +1504,11 @@ static int decode_batch_locked(b2c_decoder_t* d, const void* const* logits, cons
     bool cap_ok[kNumCaps];
     for (int c = 0; c < kNumCaps; ++c) cap_ok[c] = layout_of(c, 1, false, 0).smem_bytes <= smem_budget;
     std::vector<std::vector<int>> classes;                 // fast classes (one used per call), last = general
-    bool use_v5 = false, use_lean = false;
+    bool use_v5 = false;
     int v5_top = -1, v5_variant = 0;
     auto classify = [&]() {
         classes.assign(kNumCaps + 1, std::vector<int>());
-        use_v5 = false; use_lean = false;
+        use_v5 = false;
         v5_top = -1; v5_variant = 0;
         std::vector<int> cls_of(n_utts, kNumCaps);
         int top = -1, n_fast = 0;
@@ -1576,13 +1549,6 @@ static int decode_batch_locked(b2c_decoder_t* d, const void* const* logits, cons
             }
         }
         if (const char* e = std::getenv("B200CTC_V5_VARIANT")) v5_variant = std::max(0, std::min(2, std::atoi(e)));
-        // the lean one-warp variant: more utterances than the chosen variant keeps resident, and the previous call of
-        // this configuration says that (nearly) every utterance fits 32 slots / 128 candidates / 16 tokens per frame
-        const bool no_lean = std::getenv("B200CTC_NO_LEAN") != nullptr || !env_switch("B200CTC_LEAN", B2C_DEFAULT_LEAN != 0);
-        const bool force_lean = std::getenv("B200CTC_FORCE_LEAN") != nullptr;
-        use_lean = use_v5 && opts->beam_width <= 128 &&
-                   (force_lean || (!no_lean && (hint_ok && !d->lean_bad && d->hint_utts > 0 && 20ull * d->hint_wide_utts <= d->hint_utts &&
-                                   n_fast > d->n_sm * kV5Occ[v5_variant])));
         for (int q = 0; q < n_utts; ++q) {
             const int u = order[q];             // keeps longest-first order inside every class
             classes[cls_of[u] < kNumCaps ? top : kNumCaps].push_back(u);
@@ -1635,20 +1601,14 @@ static int decode_batch_locked(b2c_decoder_t* d, const void* const* logits, cons
             kmax = std::max(kmax, h_maxk[u]);
         }
         const u64 worst_m = static_cast<u64>(W_tab) * std::min<u32>(kmax, static_cast<u32>(V));
-        ln.v5 = (use_v5 && cls < kNumCaps) ? (use_lean ? 3 : v5_variant) : -1;
-        if (ln.v5 == 3) {
-            // lean variant: 32 slots, 128 candidates, no out-of-line tier (what does not fit is handed back)
-            ln.threads = 32;
-            ln.L = make_layout(32, V, tmax, full, smem_budget, 128, 0, 1);
-            ln.L.smem_bytes = static_cast<u32>(kV5Smem[3][V <= B2C_FAST_LT ? 1 : 0]);
-            ln.per_sm = kV5Occ[3];
-        } else if (ln.v5 >= 0) {
-            // beam tables of capacity 128; the HBM tier always exists (frames with more tokens than the rings hold use it too)
+        ln.v5 = (use_v5 && cls < kNumCaps) ? v5_variant : -1;
+        if (ln.v5 >= 0) {
+            // beam tables of capacity B2C_FAST_W; the HBM tier always exists (frames with more tokens than the rings hold use it too)
             const u32 cap5 = kV5Cap[ln.v5];
-            ln.threads = kV5Threads[ln.v5];
-            // backtrack arena: fixed node ids of the frame steps below 128 * T, the out-of-line step allocates above
-            ln.L = make_layout(128, V, tmax, full, smem_budget, cap5, std::max<u64>(worst_m, cap5 + 1), B2C_FAST_NW,
-                               128ull * static_cast<u64>(std::max(tmax, 1)));
+            ln.threads = B2C_FAST_W;
+            // backtrack arena: fixed node ids of the frame steps below B2C_FAST_W * T, the out-of-line step allocates above
+            ln.L = make_layout(B2C_FAST_W, V, tmax, full, smem_budget, cap5, std::max<u64>(worst_m, cap5 + 1), B2C_FAST_NW,
+                               static_cast<u64>(B2C_FAST_W) * static_cast<u64>(std::max(tmax, 1)));
             ln.L.smem_bytes = static_cast<u32>(kV5Smem[ln.v5][V <= B2C_FAST_LT ? 1 : 0]);
             ln.per_sm = kV5Occ[ln.v5];
         } else {
@@ -1971,8 +1931,6 @@ static int decode_batch_locked(b2c_decoder_t* d, const void* const* logits, cons
         for (int q = 0; q < 7; ++q) d->tm.cand_hist[q] = ms[q];
         d->tm.inplace_frames = ms[7];
         d->tm.sorted_frames = ms[8];
-        d->hint_wide_utts = ms[9];
-        d->hint_utts = ms[10];
         d->tm.oversize_frames = 0;
         for (int q = 0; q < 6; ++q)
             if (static_cast<int>(128u << q) == d->tm.cap_candidates) d->tm.oversize_frames = ms[q];
@@ -1982,22 +1940,9 @@ static int decode_batch_locked(b2c_decoder_t* d, const void* const* logits, cons
     int* h_status = reinterpret_cast<int*>(hs + off_st);
     std::vector<int> failed;
     for (int i = 0; i < n_utts; ++i) if (h_status[i] != B2C_OK) failed.push_back(i);
-    if (use_lean && 10 * failed.size() > static_cast<size_t>(n_utts)) d->lean_bad = true;     // not worth it for this configuration
-    // retry passes: (1) utterances the lean variant handed back -> a full latency-first variant; (2) utterances whose
-    // arenas overflowed -> the general kernel with worst-case arenas
-    for (int pass = 0; pass < 2 && !failed.empty(); ++pass) {
-        bool only_slots = use_lean && pass == 0;
-        for (int i : failed) only_slots = only_slots && h_status[i] == B2C_ERR_SLOTS;
-        if (pass == 0 && !only_slots) continue;
-        Launch ln;
-        if (only_slots) {
-            use_lean = false;
-            int fast_cls = 0;
-            for (const Launch& l0 : launches) if (l0.v5 >= 0) fast_cls = l0.cls;
-            ln = plan(failed, fast_cls, false, static_cast<size_t>(n_utts));
-        } else {
-            ln = plan(failed, kNumCaps, true, static_cast<size_t>(n_utts));
-        }
+    // utterances whose arenas overflowed: decoded again by the general kernel with worst-case arenas
+    if (!failed.empty()) {
+        const Launch ln = plan(failed, kNumCaps, true, static_cast<size_t>(n_utts));
         if (ln.L.smem_bytes > d->smem_optin) return fail(B2C_E_ARG, "beam_width too large for the shared-memory selection arrays");
         if (d->d_ws.ensure(static_cast<u64>(ln.slots) * ln.L.gws_bytes)) return B2C_E_NOMEM;
         for (size_t i = 0; i < failed.size(); ++i) h_ord[n_utts + i] = failed[i];
@@ -2016,12 +1961,9 @@ static int decode_batch_locked(b2c_decoder_t* d, const void* const* logits, cons
         CUDA_OK(cudaMemcpyAsync(d->h_out_toks.p, d->d_out_toks.p, tok_bytes, cudaMemcpyDeviceToHost, st));
         CUDA_OK(cudaMemcpyAsync(d->h_out_frames.p, d->d_out_frames.p, frm_bytes, cudaMemcpyDeviceToHost, st));
         CUDA_OK(cudaStreamSynchronize(st));
-        std::vector<int> still;
-        for (int i : failed) if (h_status[i] != B2C_OK) still.push_back(i);
-        failed.swap(still);
     }
     for (int i : failed)
-        return fail(B2C_E_INTERNAL, "beam kernel workspace overflow (status " + std::to_string(h_status[i]) + ")");
+        if (h_status[i] != B2C_OK) return fail(B2C_E_INTERNAL, "beam kernel workspace overflow (status " + std::to_string(h_status[i]) + ")");
 #if defined(B2C_PHASE_CLOCKS)
     {
         u64 hc[32];

@@ -1,4 +1,4 @@
-// b200ctc -- latency-first variant of the per-utterance prefix beam search for beam_width <= WC
+// b200ctc -- latency-first variant of the per-utterance prefix beam search for beam_width <= B2C_FAST_W
 // (same algorithm and the same results as b2c_beam.h, which stays the general path).
 //
 // A C2-shaped batch (256 utterances x 1000 frames on 148 SMs) keeps every utterance resident, so the
@@ -47,7 +47,8 @@
 #define B2C_FAST_HR 32          // frame-record ring (frames)
 #define B2C_FAST_TR 8           // token ring (frames)
 #define B2C_FAST_RMAX 6         // longest run of in-place frames handled by one step (<= B2C_FAST_TR - 2)
-#define B2C_FAST_NW 4           // most warps per CTA (a CTA has WC threads: one per beam slot; per-warp slot arrays have 4 entries)
+#define B2C_FAST_W 128          // threads per CTA = beam slots (one per thread)
+#define B2C_FAST_NW (B2C_FAST_W / 32)   // warps per CTA (per-warp slot arrays have one entry each)
 
 #if defined(__CUDA_ARCH__)
 #define B2C_LAST_THREAD if (threadIdx.x == blockDim.x - 1)
@@ -67,13 +68,12 @@ constexpr u32 b2c_pt_cap_c(int W) {
     return p;
 }
 
-template <int WC>
 struct B2cFastTab {          // one beam table (same fields as B2cBeamTab)
-    double logit[WC], lm_hw[WC], pscore[WC];
-    u64 text_hash[WC], part_hash[WC], hist_hash[WC];
-    u32 text_node[WC], chain[WC];
-    int pf_s[WC], pf_e[WC];
-    u16 last_tok[WC], part_len[WC];
+    double logit[B2C_FAST_W], lm_hw[B2C_FAST_W], pscore[B2C_FAST_W];
+    u64 text_hash[B2C_FAST_W], part_hash[B2C_FAST_W], hist_hash[B2C_FAST_W];
+    u32 text_node[B2C_FAST_W], chain[B2C_FAST_W];
+    int pf_s[B2C_FAST_W], pf_e[B2C_FAST_W];
+    u16 last_tok[B2C_FAST_W], part_len[B2C_FAST_W];
 };
 
 // asynchronous global -> shared copies (LDGSTS); hostsim: plain copies
@@ -107,10 +107,10 @@ B2C_HD void b2c_cp_async_wait_all() {
 
 // LT: entries of the shared-memory label table (V <= LT: the table is resident, runs of in-place frames are
 // enabled); 0: labels are staged per frame from global memory (large alphabets)
-template <int WC, int CAP, int LT>
+template <int CAP, int LT>
 struct B2cFastSmem {
     static constexpr u32 HT = 2u * CAP;               // grouping table slots
-    static constexpr u32 PT = b2c_pt_cap_c(WC);        // history-prune table slots
+    static constexpr u32 PT = b2c_pt_cap_c(B2C_FAST_W); // history-prune table slots
     static constexpr int KR = CAP >= 1024 ? 32 : 16;   // tokens per frame the rings hold (wider frames: out-of-line step)
     static constexpr int LTN = LT > 0 ? LT : 1;
     B2cScalars sc;
@@ -125,14 +125,14 @@ struct B2cFastSmem {
 #endif
     u32 wtop[B2C_FAST_NW];                            // per warp: 1 + best rank selected this frame
     alignas(16) u64 wmax[B2C_FAST_NW];                // per warp: best score key of this frame
-    alignas(16) B2cFastTab<WC> tab[2];
+    alignas(16) B2cFastTab tab[2];
     // selection
-    u64 phk[WC];
-    u32 ord[WC], pslot[WC];
+    u64 phk[B2C_FAST_W];
+    u32 ord[B2C_FAST_W], pslot[B2C_FAST_W];
     u32 pt_idx[PT], pt_min[PT];
     alignas(16) u32 bcnt[B2C_NBUCKET];
     alignas(16) u32 bhead[B2C_NBUCKET];
-    alignas(16) u32 bpre[WC / 32][B2C_NBUCKET];
+    alignas(16) u32 bpre[B2C_FAST_NW][B2C_NBUCKET];
     // candidates
     u64 ckey[CAP];           // merge key; after phase B: order-preserving score key of group leaders, 0 otherwise
     double cfold[CAP];       // phase A: own logit sum; after phase B (leaders): merged logit_score
@@ -151,8 +151,7 @@ struct B2cFastSmem {
     u8 fall[KR];
 };
 
-template <int WC>
-B2C_HD void b2c_fast_tab_view(B2cFastTab<WC>& t, B2cBeamTab& v) {
+B2C_HD void b2c_fast_tab_view(B2cFastTab& t, B2cBeamTab& v) {
     v.logit = t.logit; v.lm_hw = t.lm_hw; v.pscore = t.pscore;
     v.text_hash = t.text_hash; v.part_hash = t.part_hash; v.hist_hash = t.hist_hash;
     v.text_node = t.text_node; v.chain = t.chain;
@@ -162,20 +161,20 @@ B2C_HD void b2c_fast_tab_view(B2cFastTab<WC>& t, B2cBeamTab& v) {
 
 // descriptor for the general helpers (b2c_utt_begin, b2c_finalize, the out-of-line slow step);
 // `slow`: hide the shared-memory tier so that the general frame step works on the HBM tier
-template <int WC, int CAP, int LT>
-B2C_HD void b2c_fast_work(B2cFastSmem<WC, CAP, LT>& S, const B2cLayout& L, u8* g, int par, bool slow, B2cWork& W) {
+template <int CAP, int LT>
+B2C_HD void b2c_fast_work(B2cFastSmem<CAP, LT>& S, const B2cLayout& L, u8* g, int par, bool slow, B2cWork& W) {
     W.sc = &S.sc;
     b2c_fast_tab_view(S.tab[par], W.cur);
     b2c_fast_tab_view(S.tab[par ^ 1], W.nxt);
     W.phk = S.phk; W.ord = S.ord; W.pslot = S.pslot;
-    W.pt_cap = B2cFastSmem<WC, CAP, LT>::PT;
+    W.pt_cap = B2cFastSmem<CAP, LT>::PT;
     W.pt_idx = S.pt_idx; W.pt_min = S.pt_min;
     W.n_bucket = B2C_NBUCKET;
     W.bcnt = S.bcnt; W.bhead = S.bhead; W.bpre = &S.bpre[0][0];
     W.stok = nullptr; W.slp = nullptr; W.sid = nullptr;
     B2cCandTier& c = W.tier_s;
     c.cap = slow ? 0u : static_cast<u32>(CAP);
-    c.ht_cap = B2cFastSmem<WC, CAP, LT>::HT;
+    c.ht_cap = B2cFastSmem<CAP, LT>::HT;
     c.ckey = S.ckey; c.cfold = S.cfold; c.cth = nullptr; c.cph = S.cph;
     c.cmeta = S.cmeta; c.cslot = S.cslot; c.cnext = S.cnext; c.clast = S.clast;
     c.ht_idx = S.ht_idx; c.ht_min = S.ht_min; c.ht_max = S.ht_max; c.ht_cnt = S.ht_cnt;
@@ -198,8 +197,8 @@ B2C_HD void b2c_fast_work(B2cFastSmem<WC, CAP, LT>& S, const B2cLayout& L, u8* g
 
 // label record of token k of the current frame: straight from the resident table (small alphabets: one more
 // dependent shared-memory load, no per-frame staging), or from the staged copy (large alphabets)
-template <int WC, int CAP, int LT>
-B2C_HD const B2cTok& b2c_fast_tok(const B2cFastSmem<WC, CAP, LT>& S, int sb, int slot, int k) {
+template <int CAP, int LT>
+B2C_HD const B2cTok& b2c_fast_tok(const B2cFastSmem<CAP, LT>& S, int sb, int slot, int k) {
     if (LT > 0) return S.ltab[S.rid[slot][k]];
     return S.stok[sb][k];
 }
@@ -274,8 +273,8 @@ B2C_HD void b2c_bucket_scan_warp_v(const u32* bcnt, u32* pre) {
 
 // candidate i (a group leader) becomes beam j of the next frame (decoder.py:452-534 metadata); called by the
 // thread that owns the candidate, inside the ranking loop
-template <int WC, int CAP, int LT>
-B2C_HD void b2c_fast_commit(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, const B2cFastTab<WC>& cur, B2cFastTab<WC>& nx,
+template <int CAP, int LT>
+B2C_HD void b2c_fast_commit(const B2cParams& P, B2cFastSmem<CAP, LT>& S, const B2cFastTab& cur, B2cFastTab& nx,
                             B2cChain* chain_arena, B2cText* text_arena, u32 text_cap, int sb, int slot, int t, u32 j, u32 i,
                             u32 last, u32 flags) {
     const u32 bk = S.cbk[last];
@@ -296,16 +295,16 @@ B2C_HD void b2c_fast_commit(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, con
     // partial_frames (decoder.py:454-461,495,513,519-523)
     const int ps0 = cur.pf_s[bl], pe0 = cur.pf_e[bl];
     int pfs, pfe;
-    if (type == 0) { pfs = ps0; pfe = (b2c_fast_tok<WC, CAP, LT>(S, sb, slot, static_cast<int>(k)).flags & B2C_TF_BLANK) ? pe0 : t + 1; }
+    if (type == 0) { pfs = ps0; pfe = (b2c_fast_tok<CAP, LT>(S, sb, slot, static_cast<int>(k)).flags & B2C_TF_BLANK) ? pe0 : t + 1; }
     else if (type == 1) { pfs = t; pfe = t + 1; }
     else if (type == 2) { pfs = -1; pfe = -1; }
     else { pfs = ps0 < 0 ? t : ps0; pfe = t + 1; }
     nx.pf_s[j] = pfs;
     nx.pf_e[j] = pfe;
-    // backtrack chain: the node of (frame t, new slot j) has the fixed id t * WC + j -- no allocation counter
+    // backtrack chain: the node of (frame t, new slot j) has the fixed id t * B2C_FAST_W + j -- no allocation counter
     u32 chain = cur.chain[bl];
     if (type != 0) {
-        const u32 id = static_cast<u32>(t) * static_cast<u32>(WC) + j;
+        const u32 id = static_cast<u32>(t) * B2C_FAST_W + j;
         B2cChain c;
         c.parent = chain;
         c.tok = static_cast<u16>(S.rid[slot][k]);
@@ -408,11 +407,11 @@ B2C_HD void b2c_sorted_counts(const double* const (&list)[NS], u32 n, const doub
 #endif
     for (int q = 0; q < NS; ++q) cnt[q] = pos[q];
 }
-// one question against the list logit[p] + lp2 computed on the fly (unit test: tests/hostsim/t_sorted_count.cpp)
-template <int WC>
+// one question against the list logit[p] + lp2 computed on the fly, n <= N (unit test: tests/hostsim/t_sorted_count.cpp)
+template <int N>
 B2C_HD u32 b2c_sorted_count(const double* logit, u32 n, double lp2, double s, bool ge) {
-    static_assert(WC <= 128, "radix search covers 128 slots");
-    double tmp[WC];
+    static_assert(N <= 128, "radix search covers 128 entries");
+    double tmp[N];
     for (u32 p = 0; p < n; ++p) tmp[p] = (logit[p] + lp2) + 0.0;
     const double* const l1[1] = {tmp};
     const double s1[1] = {ge ? s : b2c_next_up(s)};
@@ -502,12 +501,12 @@ B2C_HD void b2c_rank_list_items(const double* cf, u32 n, int K, const u32* masks
 // hold the number of slots and the best score key of the previous frame (per-warp maxima).
 // Invariants on entry: grouping table clear; prune table = entries pslot[0 .. n) iff S.holes.
 // -----------------------------------------------------------------------------------------
-template <int WC, int CAP, int LT>
-B2C_HD void b2c_fast_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, B2cChain* chain_arena, B2cText* text_arena,
+template <int CAP, int LT>
+B2C_HD void b2c_fast_step(const B2cParams& P, B2cFastSmem<CAP, LT>& S, B2cChain* chain_arena, B2cText* text_arena,
                           u32 text_cap, int par, int t, int sb, int slot, int K) {
-    typedef B2cFastSmem<WC, CAP, LT> SM;
-    B2cFastTab<WC>& cur = S.tab[par];
-    B2cFastTab<WC>& nx = S.tab[par ^ 1];
+    typedef B2cFastSmem<CAP, LT> SM;
+    B2cFastTab& cur = S.tab[par];
+    B2cFastTab& nx = S.tab[par ^ 1];
     const u32 n = b2c_max_slots(S.wtop);                       // slots of the current table (live + dead)
     const u32 M = n * static_cast<u32>(K);
     const u32 flags = S.sc.flags;
@@ -543,7 +542,7 @@ B2C_HD void b2c_fast_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, B2cCh
             // a dead beam's candidates sit in a grouping slot of their own that nobody claims: never a group leader
             // (phase B), key 0 in phase C, and never mistaken for a member of the group that owns slot 0
             if (!live) { S.cslot[i] = SM::HT; continue; }
-            const B2cTok ti = b2c_fast_tok<WC, CAP, LT>(S, sb, slot, k);
+            const B2cTok ti = b2c_fast_tok<CAP, LT>(S, sb, slot, k);
             u64 th = th0;
             u64 nph;
             u32 nplen, type;
@@ -678,10 +677,6 @@ B2C_HD void b2c_fast_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, B2cCh
                 j = jn;
             }
             if (rank >= width) continue;
-            if (WC < 128 && rank >= static_cast<u32>(WC)) {        // lean variant: more survivors than slots
-                b2c_atomic_or_u32(&S.sc.status, B2C_ERR_SLOTS);
-                continue;
-            }
             if (rank + 1 > my_top) my_top = rank + 1;
             const u32 last = S.clast[i];
             if (prune) {
@@ -747,8 +742,8 @@ B2C_HD int b2c_fast_cheap_kind(u32 flags, u32 prev_single, const B2cTok& ti) {
 
 // label record of the first token of frame f (a frame whose record is in the ring): the resident table for small
 // alphabets; with per-frame staging (LT == 0) only the CURRENT frame's record is available (stok[sb][0])
-template <int WC, int CAP, int LT>
-B2C_HD const B2cTok& b2c_fast_tok0(const B2cParams& P, const B2cFastSmem<WC, CAP, LT>& S, int f, int sb) {
+template <int CAP, int LT>
+B2C_HD const B2cTok& b2c_fast_tok0(const B2cParams& P, const B2cFastSmem<CAP, LT>& S, int f, int sb) {
     (void)P;
     if (LT > 0) return S.ltab[S.rh[f & (B2C_FAST_HR - 1)].id0];
     return S.stok[sb][0];
@@ -760,10 +755,10 @@ B2C_HD const B2cTok& b2c_fast_tok0(const B2cParams& P, const B2cFastSmem<WC, CAP
 // applied from registers.  Returns the number of frames done: R, or fewer when a check failed at frame t + r (the
 // frames before it are applied, frame t + r is left to the general step), 0 = state untouched.
 // With LM / hotwords only T0 frames are in a run: the text-level and partial-word scores of a slot are constants.
-template <int WC, int CAP, int LT>
-B2C_HD int b2c_fast_run_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, B2cChain* chain_arena, int par, int t, int sb, int R) {
+template <int CAP, int LT>
+B2C_HD int b2c_fast_run_step(const B2cParams& P, B2cFastSmem<CAP, LT>& S, B2cChain* chain_arena, int par, int t, int sb, int R) {
     constexpr int HM = B2C_FAST_HR - 1;
-    B2cFastTab<WC>& cur = S.tab[par];
+    B2cFastTab& cur = S.tab[par];
     const u32 n = b2c_max_slots(S.wtop);
     const u32 flags = S.sc.flags;
     const bool has_lm = (flags & B2C_FL_LM) != 0;
@@ -838,12 +833,12 @@ B2C_HD int b2c_fast_run_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, B2
             const B2cFrameRec h = S.rh[(t + j) & HM];
             l = l + h.lp0;
             if (!live) continue;
-            const B2cTok& ti = b2c_fast_tok0<WC, CAP, LT>(P, S, t + j, sb);
+            const B2cTok& ti = b2c_fast_tok0<CAP, LT>(P, S, t + j, sb);
             const bool blank = (ti.flags & B2C_TF_BLANK) != 0;
             if (blank || prev == ti.canon) {               // branch (i)
                 if (!blank) pfe = t + j + 1;
             } else {                                       // branch (iv): a plain character
-                const u32 id = static_cast<u32>(t + j) * static_cast<u32>(WC) + static_cast<u32>(b);
+                const u32 id = static_cast<u32>(t + j) * B2C_FAST_W + static_cast<u32>(b);
                 B2cChain c;
                 c.parent = chain;
                 c.tok = h.id0;
@@ -887,15 +882,15 @@ B2C_HD int b2c_fast_run_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, B2
 // the old order with the new fields -> in-place update.  Otherwise the state is untouched and the general step runs.
 // Scratch: S.cfold[slot] (new lm_score), S.ckey[slot] (new partial score, as bits).
 // -----------------------------------------------------------------------------------------
-template <int WC, int CAP, int LT>
-B2C_HD bool b2c_fast_scored_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, B2cChain* chain_arena, int par, int t,
+template <int CAP, int LT>
+B2C_HD bool b2c_fast_scored_step(const B2cParams& P, B2cFastSmem<CAP, LT>& S, B2cChain* chain_arena, int par, int t,
                                  int sb, int slot) {
-    B2cFastTab<WC>& cur = S.tab[par];
+    B2cFastTab& cur = S.tab[par];
     const u32 n = b2c_max_slots(S.wtop);
     const u32 flags = S.sc.flags;
     const bool has_lm = (flags & B2C_FL_LM) != 0;
     const bool holes = S.holes != 0;
-    const B2cTok ti = b2c_fast_tok<WC, CAP, LT>(S, sb, slot, 0);
+    const B2cTok ti = b2c_fast_tok<CAP, LT>(S, sb, slot, 0);
     const double p = S.rlp[slot][0];
     B2C_FOR(b, n) {
         const u64 nph = b2c_hash_append(cur.part_hash[b], ti.raw_hash, ti.raw_pow);
@@ -935,7 +930,7 @@ B2C_HD bool b2c_fast_scored_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S
         cur.pf_e[b] = t + 1;
         const bool live = !holes || S.pt_min[S.pslot[b]] == static_cast<u32>(b);
         if (!live) continue;
-        const u32 id = static_cast<u32>(t) * static_cast<u32>(WC) + static_cast<u32>(b);
+        const u32 id = static_cast<u32>(t) * B2C_FAST_W + static_cast<u32>(b);
         B2cChain cn;
         cn.parent = cur.chain[b];
         cn.tok = static_cast<u16>(S.rid[slot][0]);
@@ -964,22 +959,22 @@ B2C_HD bool b2c_fast_scored_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S
 // fold, no score buckets.  Phases: liveness masks (and release of the previous prune entries) | ranks | commit
 // (one new beam per thread) -- the third barrier is the caller's.
 // -----------------------------------------------------------------------------------------
-template <int WC, int CAP, int LT>
-B2C_HD bool b2c_fast_sorted_ok(const B2cParams& P, const B2cFastSmem<WC, CAP, LT>& S, int sb, int slot, int K, u32 prev_single) {
+template <int CAP, int LT>
+B2C_HD bool b2c_fast_sorted_ok(const B2cParams& P, const B2cFastSmem<CAP, LT>& S, int sb, int slot, int K, u32 prev_single) {
     if (prev_single == B2C_NONE_U32 || K < 2 || K > B2C_SORTED_MAXK || P.has_dup_labels) return false;
     if (S.sc.flags & (B2C_FL_PSCORE | B2C_FL_BPE)) return false;
     u32 fl = 0;
-    for (int k = 0; k < K; ++k) fl |= b2c_fast_tok<WC, CAP, LT>(S, sb, slot, k).flags;
+    for (int k = 0; k < K; ++k) fl |= b2c_fast_tok<CAP, LT>(S, sb, slot, k).flags;
     return (fl & B2C_TF_SPACE) == 0;
 }
 
 // returns false (state untouched) when the best score is not finite
-template <int WC, int CAP, int LT>
-B2C_HD bool b2c_fast_sorted_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S, B2cChain* chain_arena, int par, int t,
+template <int CAP, int LT>
+B2C_HD bool b2c_fast_sorted_step(const B2cParams& P, B2cFastSmem<CAP, LT>& S, B2cChain* chain_arena, int par, int t,
                                  int sb, int slot, int K, u32 prev_single) {
-    typedef B2cFastSmem<WC, CAP, LT> SM;
-    B2cFastTab<WC>& cur = S.tab[par];
-    B2cFastTab<WC>& nx = S.tab[par ^ 1];
+    typedef B2cFastSmem<CAP, LT> SM;
+    B2cFastTab& cur = S.tab[par];
+    B2cFastTab& nx = S.tab[par ^ 1];
     const u32 n = b2c_max_slots(S.wtop);
     const bool prune = (S.sc.flags & B2C_FL_PRUNE) != 0;
     const bool holes = S.holes != 0;
@@ -999,7 +994,7 @@ B2C_HD bool b2c_fast_sorted_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S
 #if !defined(__CUDA_ARCH__)
     for (int w = 0; w < B2C_FAST_NW; ++w) S.wmask[w] = 0;
 #endif
-    B2C_FOR(b, WC) {
+    B2C_FOR(b, B2C_FAST_W) {
         bool live = static_cast<u32>(b) < n;
         if (live && holes) {
             const u32 ps = S.pslot[b];
@@ -1027,10 +1022,6 @@ B2C_HD bool b2c_fast_sorted_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S
         // candidate (b, k) takes rank `rank` (if it is inside the beam width)
         auto place = [&](u32 b, u32 k, u32 rank) {
             if (rank >= width) return;
-            if (WC < 128 && rank >= static_cast<u32>(WC)) {        // lean variant: more survivors than slots
-                b2c_atomic_or_u32(&S.sc.status, B2C_ERR_SLOTS);
-                return;
-            }
             S.ord[rank] = b | (k << 16);
             if (rank + 1 > my_top) my_top = rank + 1;
         };
@@ -1082,7 +1073,7 @@ B2C_HD bool b2c_fast_sorted_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S
     B2C_FOR(r, n_new) {
         const u32 e = S.ord[r];
         const u32 b = e & 0xFFFFu, k = e >> 16;
-        const B2cTok ti = b2c_fast_tok<WC, CAP, LT>(S, sb, slot, static_cast<int>(k));
+        const B2cTok ti = b2c_fast_tok<CAP, LT>(S, sb, slot, static_cast<int>(k));
         const bool blank = (ti.flags & B2C_TF_BLANK) != 0;
         const bool same = blank || ti.canon == prev_single;                      // branch (i), else branch (iv)
         const u64 ph = cur.part_hash[b];
@@ -1096,7 +1087,7 @@ B2C_HD bool b2c_fast_sorted_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S
             nph = b2c_hash_append(ph, ti.raw_hash, ti.raw_pow);
             nplen = plen + ti.raw_nchars;
             pfs = ps0 < 0 ? t : ps0;
-            const u32 id = static_cast<u32>(t) * static_cast<u32>(WC) + static_cast<u32>(r);
+            const u32 id = static_cast<u32>(t) * B2C_FAST_W + static_cast<u32>(r);
             B2cChain c;
             c.parent = chain;
             c.tok = static_cast<u16>(S.rid[slot][k]);
@@ -1143,11 +1134,11 @@ B2C_HD bool b2c_fast_sorted_step(const B2cParams& P, B2cFastSmem<WC, CAP, LT>& S
 
 // squeeze the dead slots out of the current table (into the other one: the caller flips its parity) and
 // leave the state the general helpers expect: sc.n_beams / sc.prev_max set, prune table clear
-template <int WC, int CAP, int LT>
-B2C_HDN void b2c_fast_compact(B2cFastSmem<WC, CAP, LT>* Sp, int par) {
-    B2cFastSmem<WC, CAP, LT>& S = *Sp;
-    const B2cFastTab<WC>& cur = S.tab[par];
-    B2cFastTab<WC>& nx = S.tab[par ^ 1];
+template <int CAP, int LT>
+B2C_HDN void b2c_fast_compact(B2cFastSmem<CAP, LT>* Sp, int par) {
+    B2cFastSmem<CAP, LT>& S = *Sp;
+    const B2cFastTab& cur = S.tab[par];
+    B2cFastTab& nx = S.tab[par ^ 1];
     const u32 n = b2c_max_slots(S.wtop);
     const bool holes = S.holes != 0;
     const double prev_max = b2c_key_f64(b2c_max_slots(S.wmax));
@@ -1186,10 +1177,10 @@ B2C_HDN void b2c_fast_compact(B2cFastSmem<WC, CAP, LT>* Sp, int par) {
 
 // A frame that does not fit the shared-memory tier (or the token stage): the general step on the
 // HBM tier, out of line, with its own descriptor.  Restores the invariants of b2c_fast_step.
-template <int WC, int CAP, int LT>
+template <int CAP, int LT>
 B2C_HDN void b2c_fast_slow_step(B2cParams P, B2cLayout L, u8* smem, u8* g, int par, int t, const u32* tk_id, const double* tk_lp,
                                 int K, int K_next) {
-    B2cFastSmem<WC, CAP, LT>& S = *reinterpret_cast<B2cFastSmem<WC, CAP, LT>*>(smem);
+    B2cFastSmem<CAP, LT>& S = *reinterpret_cast<B2cFastSmem<CAP, LT>*>(smem);
     B2cWork W;
     b2c_fast_work(S, L, g, par, true, W);
     const u32 M = S.sc.n_beams * static_cast<u32>(K);
@@ -1228,9 +1219,9 @@ B2C_HDN void b2c_fast_slow_step(B2cParams P, B2cLayout L, u8* smem, u8* g, int p
 // An iteration handles frame t, or a run of R in-place frames t .. t+R-1 with t + R < tv (the label records of
 // frame t + R are staged during the iteration, which needs its ids in the ring).
 // -----------------------------------------------------------------------------------------
-template <int WC, int CAP, int LT>
+template <int CAP, int LT>
 B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
-    typedef B2cFastSmem<WC, CAP, LT> SM;
+    typedef B2cFastSmem<CAP, LT> SM;
     constexpr int KR = SM::KR;
     constexpr int HM = B2C_FAST_HR - 1, TM = B2C_FAST_TR - 1;
     SM& S = *reinterpret_cast<SM*>(smem);
@@ -1242,7 +1233,6 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
     const int V = A.P.V;
     u32 st_over[6] = {0, 0, 0, 0, 0, 0};    // candidate-count histogram of the fast frames (last thread's copy counts)
     u32 st_frames = 0, st_inplace = 0, st_sorted = 0;
-    u32 st_wide_utts = 0, st_utts = 0;      // utterances a one-warp CTA (32 slots, 128 candidates, 16 tokens) could NOT hold
     B2C_LEADER {
         for (int q = 0; q < 6; ++q) S.sc.m_over[q] = 0;
         S.sc.m_frames = 0;
@@ -1326,8 +1316,8 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
             for (int c = 0; c < B2C_FAST_NW; ++c) { S.wmax[c] = 0; S.wtop[c] = 0; S.wmask[c] = 0; }
             S.wtop[0] = 1;
             S.wmax[0] = b2c_f64_key(0.0);
-            // backtrack nodes of the frame steps have fixed ids below WC * T; the out-of-line step allocates above
-            S.sc.chain_used = static_cast<u32>(WC) * static_cast<u32>(Tn);
+            // backtrack nodes of the frame steps have fixed ids below B2C_FAST_W * T; the out-of-line step allocates above
+            S.sc.chain_used = B2C_FAST_W * static_cast<u32>(Tn);
         }
         }
         B2C_SYNC();                                             // records visible
@@ -1350,7 +1340,6 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
         }
         B2C_SYNC();
         int t = ts;
-        bool wide_utt = false;
 #if defined(__CUDACC__)
 #pragma unroll 1
 #endif
@@ -1362,25 +1351,16 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
             // ---- what kind of step, and how many frames it covers ------------------------------------------
             const u32 Mq = b2c_max_slots(S.wtop) * static_cast<u32>(K);
             const bool oversize = Mq > static_cast<u32>(CAP) || K > KR;
-            wide_utt = wide_utt || Mq > 128u || K > 16 || Mq > 32u * static_cast<u32>(K);
-            if (WC < 128 && (oversize || S.sc.status != B2C_OK)) {
-                // lean variant (one warp, WC slots): no out-of-line tier and no room for more survivors -- the
-                // utterance is handed back with an error status and decoded again by the full variant (host retry pass)
-                B2C_SYNC();
-                B2C_LEADER { S.sc.status |= B2C_ERR_SLOTS; }
-                B2C_SYNC();
-                break;
-            }
             int kind = B2C_CHEAP_NO;
             int R = 1;
             if (!oversize && K == 1 && prev_single != B2C_NONE_U32) {
-                kind = b2c_fast_cheap_kind(flags, prev_single, b2c_fast_tok0<WC, CAP, LT>(A.P, S, t, sb));
+                kind = b2c_fast_cheap_kind(flags, prev_single, b2c_fast_tok0<CAP, LT>(A.P, S, t, sb));
                 if (LT > 0 && (kind == B2C_CHEAP_T0 || kind == B2C_CHEAP_T3)) {
                     // extend the run while the next frames are in-place frames too; frame t + R must have its token
                     // list in the ring (its label records are staged during this iteration)
                     int lim = te - t < B2C_FAST_RMAX ? te - t : B2C_FAST_RMAX;
                     if (tv < te && tv - 1 - t < lim) lim = tv - 1 - t;
-                    u32 pc = b2c_fast_tok0<WC, CAP, LT>(A.P, S, t, sb).canon;
+                    u32 pc = b2c_fast_tok0<CAP, LT>(A.P, S, t, sb).canon;
                     while (R < lim) {
                         const B2cFrameRec hn = S.rh[(t + R) & HM];
                         if (hn.cnt != 1) break;
@@ -1433,26 +1413,26 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
                 const u64 base_a = (f0 + static_cast<u64>(t & ~(B2C_RUN - 1))) * static_cast<u64>(V) + h.off;
                 const int K_next = t + 1 < te ? static_cast<int>(S.rh[(t + 1) & HM].cnt) : 1;
                 // the general step wants a dense table: squeeze first (the squeezed table is the other one)
-                b2c_fast_compact<WC, CAP, LT>(&S, par);
+                b2c_fast_compact<CAP, LT>(&S, par);
                 par ^= 1;
-                b2c_fast_slow_step<WC, CAP, LT>(A.P, L, smem, g, par, t, A.tok_ids + base_a, A.tok_lp + base_a, K, K_next);
+                b2c_fast_slow_step<CAP, LT>(A.P, L, smem, g, par, t, A.tok_ids + base_a, A.tok_lp + base_a, K, K_next);
                 done_frames = 1;
             } else {
                 B2C_LAST_THREAD {
                     for (int c = 0; c < 6; ++c) st_over[c] += (Mq > (128u << c)) ? 1u : 0u;
                 }
                 if (kind == B2C_CHEAP_T3P) {
-                    in_place = b2c_fast_scored_step<WC, CAP, LT>(A.P, S, chain_arena, par, t, sb, slot);
+                    in_place = b2c_fast_scored_step<CAP, LT>(A.P, S, chain_arena, par, t, sb, slot);
                     done_frames = in_place ? 1 : 0;
                 } else if (kind != B2C_CHEAP_NO) {
-                    done_frames = b2c_fast_run_step<WC, CAP, LT>(A.P, S, chain_arena, par, t, sb, R);
+                    done_frames = b2c_fast_run_step<CAP, LT>(A.P, S, chain_arena, par, t, sb, R);
                     in_place = done_frames > 0;
                 }
                 if (in_place) {
                     B2C_LAST_THREAD { st_inplace += static_cast<u32>(done_frames); }
                     B2C_FMARK(5);
-                } else if (kind == B2C_CHEAP_NO && b2c_fast_sorted_ok<WC, CAP, LT>(A.P, S, sb, slot, K, prev_single)) {
-                    if (b2c_fast_sorted_step<WC, CAP, LT>(A.P, S, chain_arena, par, t, sb, slot, K, prev_single)) {
+                } else if (kind == B2C_CHEAP_NO && b2c_fast_sorted_ok<CAP, LT>(A.P, S, sb, slot, K, prev_single)) {
+                    if (b2c_fast_sorted_step<CAP, LT>(A.P, S, chain_arena, par, t, sb, slot, K, prev_single)) {
                         done_frames = 1;
                         B2C_LAST_THREAD { ++st_sorted; }
                         B2C_FMARK(7);
@@ -1462,7 +1442,7 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
 #if defined(B2C_PHASE_CLOCKS) && defined(__CUDA_ARCH__)
                     const long long c0 = clock64();
 #endif
-                    b2c_fast_step<WC, CAP, LT>(A.P, S, chain_arena, text_arena, text_cap, par, t, sb, slot, K);
+                    b2c_fast_step<CAP, LT>(A.P, S, chain_arena, text_arena, text_cap, par, t, sb, slot, K);
 #if defined(B2C_PHASE_CLOCKS) && defined(__CUDA_ARCH__)
                     if (threadIdx.x == 0) {      // general frames by token count: cycles in 9..11, frames in 12..14
                         const int cls = K == 1 ? 0 : (K == 2 ? 1 : 2);
@@ -1476,7 +1456,7 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
             }
             // after a single-token frame every beam ends in that token (precondition of the in-place steps)
             const int t_last = t + done_frames - 1;
-            if (done_frames == 1) prev_single = (K == 1) ? static_cast<u32>(b2c_fast_tok0<WC, CAP, LT>(A.P, S, t, sb).canon) : B2C_NONE_U32;
+            if (done_frames == 1) prev_single = (K == 1) ? static_cast<u32>(b2c_fast_tok0<CAP, LT>(A.P, S, t, sb).canon) : B2C_NONE_U32;
             else prev_single = static_cast<u32>(S.ltab[S.rh[t_last & HM].id0].canon);
             // ---- label records of the next frame's tokens (its ids are in the ring: t + done_frames < tv) ------
             const int tn = t + done_frames;
@@ -1542,10 +1522,6 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
                 }
             }
         }
-        B2C_LAST_THREAD {
-            ++st_utts;
-            st_wide_utts += wide_utt ? 1u : 0u;
-        }
         if (chunked && te < Tn) {      // more frames in a later launch: park the state
             const u32* const sw = reinterpret_cast<const u32*>(smem);
             B2C_FOR(i, SAVE_WORDS) { parked[i] = sw[i]; }
@@ -1569,7 +1545,7 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
         O.states = A.out_states + static_cast<u64>(u) * ob;
         O.aux = nullptr;
         O.states_x = nullptr;
-        b2c_fast_compact<WC, CAP, LT>(&S, par);
+        b2c_fast_compact<CAP, LT>(&S, par);
         par ^= 1;
         {
             B2cWork W;
@@ -1585,8 +1561,6 @@ B2C_HD void b2c_beam_block_fast(const B2cBeamArgs& A, int slot_cta, u8* smem) {
             if (st_frames) b2c_atomic_add_u32(A.m_stats + 6, st_frames);
             if (st_inplace) b2c_atomic_add_u32(A.m_stats + 7, st_inplace);
             if (st_sorted) b2c_atomic_add_u32(A.m_stats + 8, st_sorted);
-            if (st_wide_utts) b2c_atomic_add_u32(A.m_stats + 9, st_wide_utts);
-            if (st_utts) b2c_atomic_add_u32(A.m_stats + 10, st_utts);
         }
         B2C_LEADER {   // frames that took the general step counted themselves in shared memory
             for (int c = 0; c < 6; ++c)

@@ -262,5 +262,4 @@ struct B2cStreamUtt { u32 beam_off, n_beams; int t0; u32 pad; };   // t0: proces
 
 // status codes written per utterance
 enum { B2C_OK = 0, B2C_ERR_CHAIN_FULL = 1, B2C_ERR_TEXT_FULL = 2, B2C_ERR_CAND_FULL = 3,
-       B2C_ERR_SLOTS = 4,
-       B2C_ERR_GATE = 8 };      // a gated launch waited too long for the streaming stage of its next chunk (host: plain call)     // the lean (one-warp) variant ran out of beam slots / candidates: decode again with the full one
+       B2C_ERR_GATE = 8 };      // a gated launch waited too long for the streaming stage of its next chunk (host: plain call)

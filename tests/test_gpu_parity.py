@@ -468,7 +468,6 @@ def test_gpu_kenlm_binary_equals_arpa(pkg, tmp_path):
 
 
 def test_gpu_pipelined_host_batches(pkg, orc, monkeypatch):
-    monkeypatch.setenv("B200CTC_PIPELINE", "1")
     monkeypatch.setenv("B200CTC_PIPELINE_ALL", "1")        # also compute-bound calls (by default only copy-bound ones)
     """Pipelined calls on the device: a [B, T, V] float32 host block is cut into chunks along T, chunk c+1 crosses PCIe
     while chunk c runs through the lane-per-row streaming kernel and a chunked launch of the beam kernel (state parked
